@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the NHD placement hot path (contract: see the task's bench.py section).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...        (N > 1, one rank per GPU)
 
 A *step* is one pass of the hot path over one batch: 4 096 pending pods scheduled, with the
@@ -273,6 +273,26 @@ def python_reference_baseline(recs, speed, pods, now, n_pods=8):
         return {'error': str(e)[:200]}
 
 
+def dump_outputs(out_dir, bindings, nodes):
+    """One float64 .npy per field of the bindings (bindings_<field>) and of the node records the step left on the
+    device (nodes_<field>), so that two builds can be compared output for output.  A 64-bit integer field becomes
+    its [low, high] 32-bit words on a last axis of 2: float64 holds those exactly."""
+    out = {}
+    for prefix, arr in (('bindings', bindings), ('nodes', nodes)):
+        for name in arr.dtype.names:
+            if name == 'pad_':
+                continue
+            a = np.ascontiguousarray(arr[name])
+            if a.dtype.kind in 'iu' and a.dtype.itemsize == 8:
+                a = a.view('<u4').reshape(a.shape + (2,))
+            out[f'{prefix}_{name}'] = a.astype(np.float64)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= 64 << 20, f'outputs to dump are {total} bytes'
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 def run_reference_arm(args, rank):
     """CPU arm: the oracle port of the reference path on the host cores.  The reference itself is one
     Python thread (NHDScheduler.py:43); its per-pod walk over all nodes is independent per node, so the
@@ -316,6 +336,8 @@ def main():
     ap.add_argument('--cpu-sample-pods', type=int, default=128)
     ap.add_argument('--no-extra', action='store_true', help='skip the side workloads (config 5, heterogeneous, moving clock)')
     ap.add_argument('--stop-after-e2e', action='store_true', help='developer switch: print value / e2e / clocks only and stop')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step computed (bindings, final node records) to DIR/<name>.npy')
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl != 'reference' else args.warmup
 
@@ -395,6 +417,8 @@ def main():
     wall_s = time.perf_counter() - t_wall0
     clocks = sampler.stop() if rank == 0 else None
     bindings = solver.fetch_bindings()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, bindings, solver.read_nodes())
     n_types = t['n_types']
 
     step_ms = float(np.sum(phase['total_ms']))

@@ -1,9 +1,32 @@
 """Shared test helpers: run a packed scenario through the oracle / the host-emulated core."""
 import ctypes
+import hashlib
+import json
+import os
 
 import numpy as np
 
 from nhd_b200 import wire
+
+FROZEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'frozen')
+
+
+def digest(x):
+    """Short fingerprint of bytes, of an array's bytes or of a JSON value (dict key order ignored, as by ==).  The
+    frozen reference outcomes (golden/frozen, golden/make_frozen_golden.py) keep large values in this form."""
+    if isinstance(x, bytes):
+        raw = x
+    elif isinstance(x, np.ndarray):
+        raw = np.ascontiguousarray(x).tobytes()
+    else:
+        raw = json.dumps(x, sort_keys=True, separators=(',', ':')).encode()
+    return hashlib.sha256(raw).hexdigest()[:16]
+
+
+def frozen(name):
+    """What the unmodified reference computed for a test module's cases (golden/make_frozen_golden.py)."""
+    with open(os.path.join(FROZEN, name + '.json')) as f:
+        return json.load(f)
 
 
 def emu_solve(emu, recs, speed_table, pods, now, bw=0.9, min_busy=30.0, two_stage=False):

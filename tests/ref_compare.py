@@ -7,7 +7,7 @@ import io
 import numpy as np
 
 from nhd_b200 import packing, wire
-from tests import scenarios
+from tests import helpers, scenarios
 
 _REF_STATUS = {'none': (wire.NO_CANDIDATE, wire.BAD_MAP_TYPE), 'placed': (wire.PLACED,),
                'assign_failed': (wire.ASSIGN_FAILED, wire.REF_WOULD_CRASH), 'crash': (wire.REF_WOULD_CRASH,)}
@@ -97,6 +97,39 @@ def diff_outcome(ref_o, b):
         for k in ('cores', 'gpu_index', 'nidx'):
             if ref_o[k] != bd[k]:
                 errs.append(f"{k} ref={ref_o[k]} got={bd[k]}")
+    return errs
+
+
+def compared_fields(status, d):
+    """The fields diff_outcome compares for a reference outcome of this status, taken from d (a reference
+    outcome or a binding_dict)."""
+    if status == 'none':
+        return None
+    keys = ('node', 'mapping') + (('cores', 'gpu_index', 'nidx') if status == 'placed' else ())
+    return {k: d.get(k) for k in keys}
+
+
+def freeze_outcomes(outs):
+    """A stream of reference outcomes as [one letter per pod for its status (n)one / (p)laced / (a)ssign_failed /
+    (c)rash, digest of the fields diff_outcome compares, pod after pod]."""
+    return [''.join(o['status'][0] for o in outs),
+            helpers.digest([compared_fields(o['status'], o) for o in outs])]
+
+
+def diff_frozen_outcomes(frozen, bindings):
+    """diff_outcome over a stream kept by freeze_outcomes."""
+    letters, want = frozen
+    status_of = {s[0]: s for s in _REF_STATUS}
+    if len(letters) != len(bindings):
+        return [f'{len(bindings)} bindings for {len(letters)} reference outcomes']
+    errs, got = [], []
+    for i, (c, b) in enumerate(zip(letters, bindings)):
+        bd = binding_dict(b)
+        if bd['status'] not in _REF_STATUS[status_of[c]]:
+            errs.append(f"pod {i}: status ref={status_of[c]} got={wire.STATUS_NAMES.get(bd['status'])}")
+        got.append(compared_fields(status_of[c], bd))
+    if not errs and helpers.digest(got) != want:
+        errs.append(f'nodes / mappings / cores / GPUs / NICs are not what the reference chose: {got}')
     return errs
 
 

@@ -314,6 +314,23 @@ def drop_speed_residue(doc, names):
     return doc
 
 
+def fingerprint(doc, names=()):
+    """A state document with its bulk replaced by digests (tests.helpers.digest): one per Kubernetes record
+    kind, for pod_state, for all nodes and for the RPC answers, all without the fields drop_speed_residue
+    drops, and one per node for those fields (its NodeNic.speed_used and the nicstats of its RPC answer
+    rows), left out for the nodes in ``names``.  Two documents compare equal after drop_speed_residue(...,
+    names) exactly when their fingerprints with those names do."""
+    from tests.helpers import digest
+    bare = drop_speed_residue(doc, list(doc['nodes']))
+    rows = [r for ans in doc['rpc'] if isinstance(ans, list) for r in ans if isinstance(r, dict)]
+    residue = {n: digest([st.get('speed_used'), [r.get('nicstats') for r in rows if r.get('name') == n]])
+               for n, st in doc['nodes'].items() if n not in names}
+    k8s = bare['k8s']
+    return {'k8s': {k: digest(v) for k, v in k8s.items()} if isinstance(k8s, dict) else digest(k8s),
+            'pod_state': digest(bare['pod_state']), 'failed_schedule_count': bare['failed_schedule_count'],
+            'nodes': digest(bare['nodes']), 'rpc': digest(bare['rpc']), 'residue': residue}
+
+
 def run_mirror_loop(script, solver_factory=None):
     """Like run_mirror, but through ``nhd_b200.NHDScheduler.run()`` — the thread function with its queue
     polling and idle counting — fed by the same fake queues that drive the reference's ``run()``."""

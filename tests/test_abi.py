@@ -111,9 +111,12 @@ def test_emulated_test_build_is_refused_by_the_loader():
     """A CPU-emulated build of the library (tests/emu) must never stand in for the CUDA library by accident."""
     import subprocess
     import sys
-    emu = os.path.join(ROOT, 'tests', 'emu', '_emu_cuda.so')
-    if not os.path.exists(emu):
-        pytest.skip('emulated library not built yet (tests/test_emulated_device.py builds it)')
+    sys.path.insert(0, os.path.join(ROOT, 'tests', 'emu'))
+    try:
+        import build_emu_cuda
+    finally:
+        sys.path.pop(0)
+    emu = build_emu_cuda.build()
     code = ('from nhd_b200 import _lib\n'
             'try:\n    _lib.load(); print("LOADED")\n'
             'except RuntimeError as e:\n    print("REFUSED" if "CPU-emulated" in str(e) else "OTHER")\n')

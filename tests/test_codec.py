@@ -4,8 +4,9 @@
 ``magicattr`` under ``oracle/_shim`` — parity of the libconfig *text layout* with the real package is
 therefore unpinned, see DESIGN 8.4; parity of everything the reference class itself computes is pinned).
 
-* live: random Triad configs (``tests/triad_cfg.py``) through both — parsed topology, rewritten
-  config text after a placement, GPU-map annotation, re-parse with the network section; broken configs;
+* generated: random Triad configs (``tests/triad_cfg.py``) — parsed topology, rewritten config text
+  after a placement, GPU-map annotation, re-parse with the network section; broken configs — against
+  digests of the reference's outcomes (``tests/golden/frozen/codec.json``, ``make_frozen_golden.py``);
 * frozen: ``tests/golden/codec/cases.json`` made from the reference by ``make_codec_golden.py``;
 * properties of the libconfig reader / writer on their own (round trip, number forms, escapes, paths).
 """
@@ -17,8 +18,8 @@ import pytest
 
 from nhd_b200 import libconfig
 from nhd_b200.TriadCfgParser import TriadCfgParser
+from tests import helpers
 from tests import triad_cfg as T
-from tests.conftest import has_reference
 
 GOLDEN = os.path.join(os.path.dirname(__file__), 'golden', 'codec', 'cases.json')
 
@@ -133,29 +134,30 @@ def test_codec_reproduces_golden():
     assert kinds['topology'] > 80 and kinds['none'] > 20 and kinds['raises'] > 5, kinds
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not has_reference(), reason='needs /root/reference (build container)')
-def test_codec_matches_live_reference():
-    from oracle import ref_sched_loader
-    Ref = ref_sched_loader.load_codec().codec.TriadCfgParser
+def generated_cases():
+    """(seed, config text, broken variants of it) in the order the frozen outcomes follow."""
     rng = np.random.default_rng(77)
-    n = texts = 0
     for seed in range(120):
         pod = T.codec_pod(rng, 'wild' if seed % 2 else 'mixed')
         text = T.pod_to_cfg(pod, rng, gpu_type=[None, 'V100', 'bogus'][seed % 3])
-        want = run_case(Ref, text, False, seed)
+        yield seed, text, broken_variants(text, rng) if seed % 4 == 0 else []
+
+
+def test_codec_matches_live_reference():
+    """Generated configs against digests (``tests.helpers.digest``) of the reference's outcomes, frozen by
+    ``tests/golden/make_frozen_golden.py``: the parsed config, the rewritten config read back with its network
+    section (a deployed pod after a restart), and broken variants."""
+    frozen = helpers.frozen('codec')
+    n = texts = 0
+    for (seed, text, broken), want in zip(generated_cases(), frozen, strict=True):
         got = run_case(TriadCfgParser, text, False, seed)
-        assert got == want, seed
-        assert want['topology'] is not None
+        assert helpers.digest(got) == want['parsed'], (seed, got)
+        assert got['topology'] is not None
         texts += 1
-        # the rewritten config, read back with its network section (a deployed pod after a restart)
-        want2 = run_case(Ref, want['cfg'], True, seed)
         got2 = run_case(TriadCfgParser, got['cfg'], True, seed)
-        assert got2 == want2 and got2['topology'] is not None, seed
+        assert helpers.digest(got2) == want['reparsed'] and got2['topology'] is not None, (seed, got2)
         ids = [c[4] for g in got2['topology']['groups'] for c in g['proc'] + g['helpers']]
         assert all(x > 0 for x in ids)                           # physical ids survived the trip
-        if seed % 4 == 0:
-            for bad in broken_variants(text, rng):
-                assert run_case(TriadCfgParser, bad, False, seed) == run_case(Ref, bad, False, seed), (seed, bad[:80])
-                n += 1
+        assert [helpers.digest(run_case(TriadCfgParser, bad, False, seed)) for bad in broken] == want['broken'], seed
+        n += len(broken)
     assert texts == 120 and n > 200

@@ -11,7 +11,7 @@ import pytest
 from nhd_b200 import Node as mirror_node
 from nhd_b200 import packing, wire
 from nhd_b200.ingest import LabelError, LabelIngest
-from tests import conftest, scenarios
+from tests import helpers, scenarios
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'ingest', 'cases.json')
 
@@ -43,15 +43,22 @@ def _object_path(node_mod, case, layout):
     return 'ok', rec, n
 
 
-def _check_aux(case, rec, aux, n):
-    assert int(aux['data_vlan']) == n.data_vlan
-    assert int(aux['res_hugepages_gb']) == n.mem.res_hugepages_gb
-    assert int(aux['n_reserved_cores']) == len(n.reserved_cores)
-    assert aux['gpu_device_id'][:len(n.gpus)].tolist() == [g.device_id for g in n.gpus]
-    assert (aux['gpu_device_id'][len(n.gpus):] == -1).all()
+def aux_of(n):
+    """What the side outputs of the native ingest must say about a parsed Node object."""
+    return {'data_vlan': n.data_vlan, 'res_hugepages_gb': n.mem.res_hugepages_gb,
+            'n_reserved_cores': len(n.reserved_cores), 'gpu_device_id': [g.device_id for g in n.gpus],
+            'nic_ifname': [x.ifname for x in n.nics]}
+
+
+def native_aux(case, rec, aux):
+    """aux_of for the side outputs of the native ingest of an accepted case."""
+    n_gpus, n_nics = int(rec['n_gpus']), int(rec['n_nics'])
+    assert (aux['gpu_device_id'][n_gpus:] == -1).all()
     keys = list(case['labels'].keys())
-    assert [keys[i].split('.')[4] for i in aux['nic_label'][:len(n.nics)]] == [x.ifname for x in n.nics]
     assert keys[int(aux['gw_label'])] == 'DATA_DEFAULT_GW'
+    return {'data_vlan': int(aux['data_vlan']), 'res_hugepages_gb': int(aux['res_hugepages_gb']),
+            'n_reserved_cores': int(aux['n_reserved_cores']), 'gpu_device_id': aux['gpu_device_id'][:n_gpus].tolist(),
+            'nic_ifname': [keys[i].split('.')[4] for i in aux['nic_label'][:n_nics]]}
 
 
 def test_golden_cases_from_the_reference():
@@ -95,7 +102,7 @@ def test_native_ingest_matches_mirror_objects(flavor):
             assert kind == okind, (seed, nd['name'])
             if kind == 'ok':
                 assert rec.tobytes() == orec.tobytes(), (seed, nd['name'])
-                _check_aux(case, rec, aux, n)
+                assert native_aux(case, rec, aux) == aux_of(n), (seed, nd['name'])
                 n_ok += 1
     assert n_ok > 80
     assert ing.speed_table().tolist() == layout.speed_table().tolist()
@@ -149,28 +156,27 @@ def test_batch_ingest_brings_a_cluster_up_like_build_initial_node_list():
         assert recs[i].tobytes() == r.tobytes(), i
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not conftest.has_reference(), reason='reference not present on this machine')
-def test_fuzzed_labels_against_the_live_reference():
-    """Seeded damage to valid label dictionaries: the native parser and the unmodified reference must agree on
-    accept / return False / raise / beyond-limits, and on every byte of the accepted records."""
-    from oracle import ref_loader
+def fuzzed_cases():
     from tests.golden import make_ingest_golden as mk
-    ref = ref_loader.load()
-    rng = random.Random(5)
-    cases = mk.mutations(rng, 400)
-    ing, layout = LabelIngest(), packing.ClusterLayout()
+    return mk.mutations(random.Random(5), 400)
+
+
+def test_fuzzed_labels_against_the_live_reference():
+    """Seeded damage to valid label dictionaries: the native parser must do what the unmodified reference did
+    (frozen by tests/golden/make_frozen_golden.py) — accept / return False / raise / beyond-limits — and give
+    accepted records whose bytes hash as the reference's did, with the same side outputs."""
+    frozen = helpers.frozen('ingest')
+    ing = LabelIngest()
     kinds = {}
-    for case in cases:
+    for case, want in zip(fuzzed_cases(), frozen['fuzzed'], strict=True):
         kind, rec, aux = _native(ing, case)
-        okind, orec, n = _object_path(ref.node, case, layout)
-        assert kind == okind, (case['name'], kind, okind, case['labels'])
+        assert kind == want[0], (case['name'], kind, want[0], case['labels'])
         kinds[kind] = kinds.get(kind, 0) + 1
-        if kind == 'ok':
-            assert rec.tobytes() == orec.tobytes(), case['name']
-            _check_aux(case, rec, aux, n)
+        if kind == 'ok':              # digests of the record and of aux_of the reference's Node
+            assert helpers.digest(rec.tobytes()) == want[1], case['name']
+            assert helpers.digest(native_aux(case, rec, aux)) == want[2], case['name']
     assert kinds.get('ok', 0) > 100 and kinds.get('raises', 0) > 10 and kinds.get('false', 0) > 5, kinds
-    assert ing.speed_table().tolist() == layout.speed_table().tolist()
+    assert ing.speed_table().tolist() == frozen['fuzzed_speed_table']
 
 
 # ---- node statistics off packed records (SURVEY 8f row 4, the part the packed state carries) -------------
@@ -229,26 +235,24 @@ def test_node_stats_match_mirror_getters_after_scheduling(oracle_lib, flavor):
         _check_stats(final, _stats_of_objects(order))
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not conftest.has_reference(), reason='reference not present on this machine')
-def test_node_stats_match_reference_getters_after_scheduling():
-    """Same against the unmodified reference: its own scheduler loop leaves Node objects behind whose getters
-    (what GetBasicNodeStats calls, nhd/NHDScheduler.py:355-378) must agree with the packed records' counters."""
-    from oracle import ref_loader
-    ref = ref_loader.load()
-    import contextlib
-    import io
+def stats_scenarios():
     for seed, flavor in enumerate(['mixed', 'wild', 'vf', 'big', 'mixed', 'big']):
-        scn = scenarios.random_scenario(45000 + seed, n_nodes=8, n_pods=30, flavor=flavor)
-        nodes = scenarios.build_nodes(scn, ref.node)
-        matcher = ref.matcher.Matcher()
-        for pod, t in zip(scn['pods'], scn['now']):
-            top = scenarios.build_top(pod, ref.cfg)
-            with contextlib.redirect_stdout(io.StringIO()):
-                ref_loader.attempt_scheduling(ref, matcher, nodes, top, pod['groups'], t)
-        order = list(nodes.values())
-        recs = packing.pack_nodes(order, packing.ClusterLayout())
-        _check_stats(recs, _stats_of_objects(order))
+        yield seed, scenarios.random_scenario(45000 + seed, n_nodes=8, n_pods=30, flavor=flavor)
+
+
+def test_node_stats_match_reference_getters_after_scheduling(oracle_lib):
+    """Same against the unmodified reference: its own scheduler loop left Node objects behind whose getters
+    (what GetBasicNodeStats calls, nhd/NHDScheduler.py:355-378) must agree with the packed records' counters.
+    The records and the getters' answers are frozen (tests/golden/make_frozen_golden.py); the oracle must reach
+    the same records from the scenario."""
+    from tests import ref_compare
+    frozen = helpers.frozen('ingest')['stats']
+    for (seed, scn), want in zip(stats_scenarios(), frozen, strict=True):
+        recs = np.frombuffer(bytes.fromhex(want['records']), dtype=wire.NODE_DTYPE)
+        start, pods, now, layout = ref_compare.pack_scenario(scn)
+        _, final = oracle_lib.solve(start, layout.speed_table(), pods, now)
+        assert final.tobytes() == recs.tobytes(), seed
+        _check_stats(recs, want['rows'])
 
 
 @pytest.mark.parametrize('config,wild', [(4, False), (5, False), (4, True)])

@@ -3,17 +3,15 @@ generated code must be the reference's (``nhd/proto/nhd_stats.proto``), the hand
 the UNMODIFIED reference ``NHDRpcHandler`` (``nhd/NHDRpcServer.py:47-137``), and a live server on the
 loopback interface must answer the calls of the reference's ``test/RPCTest.py`` from a running scheduler,
 from the Python objects or from the solver's records."""
+import json
 import re
-import sys
 import threading
-import types
 from queue import Empty, Queue
 
 import pytest
 
 from nhd_b200 import NHDRpcServer as R
 from tests import helpers, sched_harness as H
-from tests.conftest import has_reference
 
 NODE_ROWS = [{'name': 'n0', 'freegpu': 3, 'totalgpu': 8, 'freecpu': 40, 'totalcpu': 96, 'freehuge_gb': 20,
               'totalhuge_gb': 64, 'totalpods': 3, 'active': True, 'nicstats': [[10, 20], [0, 0]]},
@@ -54,10 +52,9 @@ def _proto_fields(text):
     return out
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not has_reference(), reason='needs /root/reference (build container)')
 def test_descriptor_is_the_references_proto():
-    want = _proto_fields(open('/root/reference/nhd/proto/nhd_stats.proto').read())
+    """Against the reference's nhd/proto/nhd_stats.proto as _proto_fields reads it (golden/make_frozen_golden.py)."""
+    want = helpers.frozen('rpc')['proto']
     fd = R.file_descriptor_proto()
     assert fd.package == 'NhdStats' and fd.syntax == 'proto3'
     T = R._T
@@ -75,7 +72,7 @@ def test_descriptor_is_the_references_proto():
             fields.append((f.name, f.number, typ, f.label == T.LABEL_REPEATED))
         got['messages'][m.name] = sorted(fields, key=lambda f: f[1])
     got['rpcs'] = sorted((m.name, m.input_type.split('.')[-1], m.output_type.split('.')[-1]) for m in fd.service[0].method)
-    assert got == want
+    assert json.loads(json.dumps(got)) == want
     assert len(want['messages']) == 9 and len(want['rpcs']) == 4
 
 
@@ -97,45 +94,41 @@ def test_messages_round_trip_and_wire_format():
         pb.NICInfoBrief().used_rx = 'x'
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not has_reference(), reason='needs /root/reference (build container)')
-def test_handlers_match_the_reference_handler():
-    """The unmodified ``nhd.NHDRpcServer.NHDRpcHandler`` runs once ``nhd.proto.nhd_stats_pb2*`` (generated
-    code, absent) resolve to this module's message classes; both must build byte-identical responses."""
-    from oracle import ref_loader
-    ref_loader.load()
-    stub_pb = types.ModuleType('nhd.proto.nhd_stats_pb2')
-    for k in dir(R.nhd_stats_pb2):
-        if not k.startswith('_'):
-            setattr(stub_pb, k, getattr(R.nhd_stats_pb2, k))
-    stub_grpc = types.ModuleType('nhd.proto.nhd_stats_pb2_grpc')
-    stub_grpc.NHDControlServicer = object
-    stub_grpc.add_NHDControlServicer_to_server = R.add_NHDControlServicer_to_server
-    pkg = types.ModuleType('nhd.proto')
-    pkg.__path__ = []
-    pkg.nhd_stats_pb2, pkg.nhd_stats_pb2_grpc = stub_pb, stub_grpc
-    sys.modules.update({'nhd.proto': pkg, 'nhd.proto.nhd_stats_pb2': stub_pb, 'nhd.proto.nhd_stats_pb2_grpc': stub_grpc})
+ANSWERS = {'TYPE_NODE_INFO': NODE_ROWS, 'TYPE_SCHEDULER_INFO': 17, 'TYPE_POD_INFO': POD_ROWS}
+CALLS = ('GetBasicNodeStats', 'GetSchedulerStats', 'GetPodStats')
+# a Gb/s that is not an integer cannot go into a uint32 field
+BAD_ANSWERS = {'TYPE_NODE_INFO': [dict(NODE_ROWS[0], nicstats=[[22.5, 0]])]}
+
+
+def handler_responses(handler_cls):
+    """call -> serialized response of a handler fed ANSWERS; 'bad' -> name of the exception BAD_ANSWERS raise."""
+    out = {}
+    for call in CALLS:
+        q = Queue()
+        _feeder(q, ANSWERS, 1)
+        out[call] = getattr(handler_cls(q), call)(R.nhd_stats_pb2.Empty(), None).SerializeToString(deterministic=True).hex()
+    q = Queue()
+    _feeder(q, BAD_ANSWERS, 1)
     try:
-        import nhd.NHDRpcServer as ref_rpc
-        answers = {'TYPE_NODE_INFO': NODE_ROWS, 'TYPE_SCHEDULER_INFO': 17, 'TYPE_POD_INFO': POD_ROWS}
-        for call in ('GetBasicNodeStats', 'GetSchedulerStats', 'GetPodStats'):
-            q1, q2 = Queue(), Queue()
-            _feeder(q1, answers, 1)
-            _feeder(q2, answers, 1)
-            want = getattr(ref_rpc.NHDRpcHandler(q1), call)(R.nhd_stats_pb2.Empty(), None)
-            got = getattr(R.NHDRpcHandler(q2), call)(R.nhd_stats_pb2.Empty(), None)
-            assert got.SerializeToString(deterministic=True) == want.SerializeToString(deterministic=True), call
-            assert got.status == R.nhd_stats_pb2.NHD_STATUS_OK
-        # a Gb/s that is not an integer cannot go into a uint32 field: both raise (the call fails)
-        bad = {'TYPE_NODE_INFO': [dict(NODE_ROWS[0], nicstats=[[22.5, 0]])]}
-        for handler_cls in (ref_rpc.NHDRpcHandler, R.NHDRpcHandler):
-            q = Queue()
-            _feeder(q, bad, 1)
-            with pytest.raises((TypeError, ValueError)):
-                handler_cls(q).GetBasicNodeStats(R.nhd_stats_pb2.Empty(), None)
-    finally:
-        for k in ('nhd.proto', 'nhd.proto.nhd_stats_pb2', 'nhd.proto.nhd_stats_pb2_grpc', 'nhd.NHDRpcServer'):
-            sys.modules.pop(k, None)
+        handler_cls(q).GetBasicNodeStats(R.nhd_stats_pb2.Empty(), None)
+        out['bad'] = None
+    except Exception as e:                                      # noqa: BLE001 - which exception is the outcome
+        out['bad'] = type(e).__name__
+    return out
+
+
+def test_handlers_match_the_reference_handler():
+    """The unmodified ``nhd.NHDRpcServer.NHDRpcHandler`` (run on this module's message classes in place of its
+    absent generated code, golden/make_frozen_golden.py) built these responses; this handler must build them
+    byte for byte, and fail the same call the same way."""
+    want = helpers.frozen('rpc')['handlers']
+    got = handler_responses(R.NHDRpcHandler)
+    assert got == want
+    assert want['bad'] in ('TypeError', 'ValueError')
+    for call in CALLS:
+        m = getattr(R.nhd_stats_pb2, {'GetBasicNodeStats': 'NodeStats', 'GetSchedulerStats': 'SchedulerStats',
+                                      'GetPodStats': 'PodStats'}[call]).FromString(bytes.fromhex(got[call]))
+        assert m.status == R.nhd_stats_pb2.NHD_STATUS_OK
 
 
 def test_handler_times_out_with_error_status():

@@ -3,9 +3,10 @@ set goes to the solver as one batch, and everything Kubernetes, ``pod_state`` an
 objects end up with must be what the UNMODIFIED reference ``nhd.NHDScheduler.run()`` leaves behind
 when it schedules the same pods one ``AttemptScheduling`` at a time.
 
-* live (build container, ``/root/reference`` present): random scripted sessions — pods appearing,
-  Kubernetes writes failing at every step the reference unwinds from, delete / create events,
-  cordon, maintenance, group changes, restarts, RPCs — played to both;
+* random scripted sessions — pods appearing, Kubernetes writes failing at every step the reference
+  unwinds from, delete / create events, cordon, maintenance, group changes, restarts, RPCs — against
+  fingerprints of the reference's end states (``tests/golden/frozen/scheduler.json``, made by
+  ``tests/golden/make_frozen_golden.py``);
 * frozen: ``tests/golden/sched/*.json`` (made by ``tests/golden/make_sched_golden.py`` from the
   reference), replayed here on CPU and, ``-m gpu``, through the CUDA solver on the B200 box.
 
@@ -20,7 +21,6 @@ import os
 import pytest
 
 from tests import helpers, sched_harness as H
-from tests.conftest import has_reference
 
 GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), 'golden', 'sched', '*.json')))
 IDS = [os.path.basename(p)[:-5] for p in GOLDEN]
@@ -62,21 +62,25 @@ def test_scheduler_cuda_reproduces_reference_sessions(path):
     assert got == want
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not has_reference(), reason='needs /root/reference (build container)')
+def flavor_scripts(flavor):
+    for seed in range(100, 112):
+        yield seed, H.random_script(seed, flavor, codec='triad' if seed % 2 else 'json')
+
+
 @pytest.mark.parametrize('flavor', ['mixed', 'vf', 'big', 'wild'])
 def test_scheduler_matches_live_reference(oracle_lib, flavor):
+    """Scripted sessions against the fingerprints (``sched_harness.fingerprint``) of the state documents the
+    reference's ``run()`` ended in, frozen by ``tests/golden/make_frozen_golden.py``."""
+    frozen = helpers.frozen('scheduler')[flavor]
     checked = binds = 0
-    for seed in range(100, 112):
-        script = H.random_script(seed, flavor, codec='triad' if seed % 2 else 'json')
-        want = H.run_reference(script)
+    for (seed, script), want in zip(flavor_scripts(flavor), frozen, strict=True):
         stats = {}
         got = H.run_mirror(script, solver_factory=helpers.OracleSolver, stats=stats)
-        want = H.drop_speed_residue(want, stats['assign_failed_nodes'])
-        got = H.drop_speed_residue(got, stats['assign_failed_nodes'])
-        assert H.first_difference(want, got) is None, (seed, flavor)
+        names = stats['assign_failed_nodes']
+        want = dict(want, residue={n: d for n, d in want['residue'].items() if n not in names})
+        assert H.first_difference(want, H.fingerprint(got, names)) is None, (seed, flavor)
         checked += 1
-        binds += len(want['k8s']['binds'])
+        binds += len(got['k8s']['binds'])
     assert checked == 12 and binds > 100
 
 
