@@ -310,6 +310,35 @@ typedef struct nhd_node_stats {
 } nhd_node_stats;
 int32_t nhd_node_stats_from_records(int32_t n, const nhd_node_rec* recs, nhd_node_stats* out);
 
+/* ---- explanation: why FindNode drops a node for a pod ------------------------------------------
+ * The reference logs, node by node, the first stage of its path that removes a node (Matcher.py INFO
+ * records); nhd_explain computes that stage for every (pod, loaded node) pair on the device.  A node
+ * gets exactly one code: the first of the list below that applies, judged on the current records at
+ * the pod's clock now[i]. */
+#define NHD_WHY_FEASIBLE        0   /* in filts[1] when SelectNode runs                (Matcher.py:393-421) */
+#define NHD_WHY_NOT_IN_GROUP    1   /* no node group in common with the pod            (NHDScheduler.py:241) */
+#define NHD_WHY_INACTIVE        2   /* in the group but not active                     (NHDScheduler.py:242-245) */
+#define NHD_WHY_MAINTENANCE     3   /* node in maintenance                             (Matcher.py:73-75) */
+#define NHD_WHY_HUGEPAGES       4   /* too few free 1 GB hugepages                     (Matcher.py:78-79) */
+#define NHD_WHY_MAP_TYPE        5   /* pod map type neither NUMA nor PCI               (Matcher.py:45-47) */
+#define NHD_WHY_BUSY            6   /* GPU pod, last deployment within MIN_BUSY_SECS   (Matcher.py:107-111) */
+#define NHD_WHY_GPU             7   /* GPU stage empty                                 (Matcher.py:132-134) */
+#define NHD_WHY_CPU             8   /* CPU stage over (G+1)-tuples empty               (Matcher.py:214-216) */
+#define NHD_WHY_NIC             9   /* NIC stage empty without the PCIe pruning        (Matcher.py:270-272) */
+#define NHD_WHY_PCIE           10   /* intersection non-empty only without the PCIe-switch pruning (Matcher.py:295-335,349-353) */
+#define NHD_WHY_NUMA           11   /* GPU / CPU / NIC NUMA tuples do not intersect    (Matcher.py:349-353) */
+#define NHD_WHY_COUNT          12
+
+/* Read-only: the records, the snapshot, a staged batch, the last bindings, nhd_read_filter and
+ * nhd_last_timing are left as they were; returns after a synchronise.  Pods are validated as
+ * nhd_stage_batch validates them.  On a world_size > 1 handle the call is local to the rank (every
+ * rank holds every record) and runs no collective.
+ *   counts     [n_pods][NHD_WHY_COUNT]: nodes per reason; each row sums to the loaded node count
+ *   first_fit  [n_pods] or NULL: the node FindNode would return now (load order), -1 if none
+ *   reasons    [n_pods][n_nodes] or NULL: the reason code of every node */
+int32_t nhd_explain(nhd_handle* h, int32_t n_pods, const nhd_pod* pods, const double* now,
+                    int32_t* counts, int32_t* first_fit, uint8_t* reasons);
+
 #ifdef __cplusplus
 }
 #endif

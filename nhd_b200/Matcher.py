@@ -218,6 +218,25 @@ class Matcher:
         mapping['_nhd_binding'] = b
         return names[int(b['node'])], mapping
 
+    def Explain(self, nl, top, pod_groups: Iterable[str] = None, now: float = None):
+        """Why ``FindNode(nl, top)`` would drop each node of ``nl`` now — what the reference logs node by node
+        (``Matcher.py:74-353``) — without placing anything.  Returns ``(nodename or None, {node name: reason name})``
+        with the names of ``wire.WHY_NAMES``; the first element is what ``FindNode`` returns first on the same
+        state."""
+        if len(nl) == 0:
+            return None, {}
+        names, nodes, solver = self._load(nl)
+        pod = packing.pack_pod(top, [], self._layout)
+        if pod_groups is None:
+            pod['group_mask'] = np.uint64(0xFFFFFFFFFFFFFFFF)
+        else:
+            pod['group_mask'] = self._layout.groups_mask(pod_groups, create=False)
+        now = time.monotonic() if now is None else now
+        _, first, reasons = solver.explain(pod.reshape(1), [now], detail=True)
+        index = self._cl.index
+        why = {n: wire.WHY_NAMES[int(reasons[0, index[n]])] for n in nl}
+        return (names[int(first[0])] if first[0] >= 0 else None), why
+
     def FindNodesBatch(self, nl, tops: Sequence, pod_groups: Sequence[Iterable[str]] = None,
                        now=None, apply: bool = True):
         """Schedule ``tops`` in order on ``nl`` (all nodes of the cluster, NOT pre-filtered:

@@ -79,6 +79,25 @@ class RpcMsgType(Enum):                         # NHDCommon.py:69-73
     TYPE_NODE_DETAIL = 4
 
 
+OUTSIDE_LIMITS = 'OUTSIDE_LIMITS'                    # failure_reasons key: active nodes beyond the packed limits
+
+
+def unschedulable_message(reasons: Dict[str, int], n_nodes: int) -> str:
+    """kube-scheduler style summary of ``{reason name: nodes}`` (``wire.WHY_NAMES`` plus ``OUTSIDE_LIMITS``), e.g.
+    ``0/12 nodes are available: 3 not in the pod's node groups, 9 too few free CPU cores.``  Reasons in code order,
+    the nodes outside the solver's limits last.  Feasible nodes can only appear when busy windows expired after the
+    pod's attempt: the message says so."""
+    parts = [f'{reasons[name]} {wire.WHY_TEXT[w]}' for w, name in enumerate(wire.WHY_NAMES)
+             if w != wire.WHY_FEASIBLE and reasons.get(name)]
+    if reasons.get(OUTSIDE_LIMITS):
+        parts.append(f"{reasons[OUTSIDE_LIMITS]} outside the solver's limits")
+    feasible = reasons.get(wire.WHY_NAMES[wire.WHY_FEASIBLE], 0)
+    head = f'{feasible}/{n_nodes} nodes are available'
+    if feasible:
+        head += ' now (busy windows expired since the attempt)'
+    return head + (': ' + ', '.join(parts) if parts else '') + '.'
+
+
 def _type_name(t) -> str:
     """Watch / RPC types may arrive as this module's enums, the reference's, or plain names."""
     return t if isinstance(t, str) else t.name
@@ -192,6 +211,16 @@ class DeviceCluster:
         self._last = (pods, np.full(len(tops), now, dtype='<f8'))
         return self._solver.solve_batch(*self._last)
 
+    def explain(self, packed: Sequence, pod_groups: Sequence[Iterable[str]], now: float) -> np.ndarray:
+        """Nodes per ``wire.WHY_*`` reason for each packed pod on the synced cluster at ``now`` (one
+        ``nhd_explain`` call; the device state is left as it is)."""
+        pods = np.zeros(len(packed), dtype=wire.POD_DTYPE)
+        for i, rec in enumerate(packed):
+            pods[i] = rec
+            pods[i]['group_mask'] = self._layout.groups_mask(pod_groups[i], create=False)
+        counts, _, _ = self._solver.explain(pods, np.full(len(packed), now, dtype='<f8'))
+        return counts
+
     def rewind(self, k: int):
         """Put the device back to the state right after pod ``k`` of the last batch (restore the
         snapshot taken before it, solve pods ``0..k`` again: the solver is deterministic)."""
@@ -224,7 +253,10 @@ class NHDScheduler:
     def __init__(self, k8s, cfg_parser: Callable, rpcq: Queue = None, solver_factory: Callable = None,
                  device: int = 0, clock: Callable[[], float] = time.monotonic,
                  wall: Callable[[], float] = time.time, node_cls=Node, logger=None,
-                 stats_from_device: bool = False):
+                 stats_from_device: bool = False, explain_failures: bool = False):
+        """``explain_failures``: after each ``CheckPendingPods`` pass, explain on the GPU why every pod that found
+        no candidate node is unschedulable (one ``Unschedulable`` Warning event per pod, counts kept in
+        ``failure_reasons``).  Off by default: the event stream is then exactly the reference's."""
         self.nodes: Dict[str, Node] = {}
         self.k8s = k8s
         self.sched_name = NHD_SCHED_NAME
@@ -241,6 +273,9 @@ class NHDScheduler:
         self.assign_failed_nodes = set()
         self.unsupported_pods = []                   # (ns, pod, why): requests beyond the packed layout's limits
         self.stats_from_device = stats_from_device
+        self.explain_failures = explain_failures
+        self.failure_reasons: Dict[tuple, Dict[str, int]] = {}   # (ns, pod) -> {reason name: nodes}, last pass
+        self._unplaced = None                        # pods of the current pass that found no node (explain_failures)
 
     # ---- small helpers --------------------------------------------------------------------
     def _info(self, msg):
@@ -506,6 +541,8 @@ class NHDScheduler:
                     rewound = True
                 results[e.key] = ok = self._finish(e, b, now)
                 self._record(e.key, ok)
+                if self._unplaced is not None and e.pobj is not None and b is not None and int(b['node']) < 0:
+                    self._unplaced.append(e)
                 if self._dirty or rewound:            # nodes changed behind the solver's back / device rewound
                     cut = e
                     break
@@ -523,6 +560,7 @@ class NHDScheduler:
         podkey = (key[0], key[1])
         if ok:
             self.pod_state[podkey] = {'state': PodStatus.POD_STATUS_SCHEDULED, 'time': self._wall(), 'uid': key[2]}
+            self.failure_reasons.pop(podkey, None)
         else:
             self._error(f'Failed scheduling pod {key[0]}.{key[1]} [{key[2]}]')
             self.pod_state[podkey] = {'state': PodStatus.POD_STATUS_FAILED, 'time': self._wall(), 'uid': '0'}
@@ -550,9 +588,40 @@ class NHDScheduler:
                     ((podkey not in self.pod_state) or
                      self.pod_state[podkey]['state'] != PodStatus.POD_STATUS_SCHEDULED))
 
-        self.ScheduleBatch(list(phase), wanted)
+        self._unplaced = [] if self.explain_failures else None
+        try:
+            self.ScheduleBatch(list(phase), wanted)
+            unplaced = self._unplaced
+        finally:
+            self._unplaced = None
+        if unplaced:
+            self._explain_unplaced(unplaced)
         # The reference's second branch (:437-440) compares the pod_state *dict* with an enum member and
         # therefore never runs; a pod reported 'Failed' keeps its resources until its delete event.
+
+    def _explain_unplaced(self, entries: Sequence[_Pending]):
+        """Why the pods of ``entries`` found no node, on the cluster as their next attempt will find it (the state
+        after the pass, at the scheduler clock now): one ``nhd_explain`` call, one ``Unschedulable`` event each."""
+        if not self.nodes:
+            return
+        self.cluster.sync(self.nodes, self._dirty)
+        self._dirty.clear()
+        counts = self.cluster.explain([e.rec for e in entries], [e.groups for e in entries], float(self._clock()))
+        outside = sum(1 for n in self.cluster.unsupported_nodes if n in self.nodes)
+        for e, row in zip(entries, counts):
+            reasons = {wire.WHY_NAMES[w]: int(c) for w, c in enumerate(row) if c}
+            if outside:
+                # inactive stubs on the device (packing.stub_record: no node group), listed for what they are
+                moved = min(outside, reasons.get('NOT_IN_GROUP', 0))
+                if moved:
+                    reasons['NOT_IN_GROUP'] -= moved
+                    if not reasons['NOT_IN_GROUP']:
+                        del reasons['NOT_IN_GROUP']
+                    reasons[OUTSIDE_LIMITS] = moved
+            ns, podname = e.key[0], e.key[1]
+            self.failure_reasons[(ns, podname)] = reasons
+            self.k8s.GeneratePodEvent(e.pobj, podname, ns, 'Unschedulable', K8SEventType.EVENT_TYPE_WARNING,
+                                      unschedulable_message(reasons, int(row.sum())))
 
     # ---- the thread function (NHDScheduler.py:443-577) ------------------------------------------------
     def Startup(self):
@@ -595,6 +664,7 @@ class NHDScheduler:
             if t == 'NHD_WATCH_TYPE_TRIAD_POD_DELETE':
                 self.ReleasePodResources(pn, ns)
                 self.pod_state.pop((ns, pn), None)
+                self.failure_reasons.pop((ns, pn), None)
             else:
                 if ((ns, pn) in self.pod_state) and \
                         (self.pod_state[(ns, pn)]['state'] == PodStatus.POD_STATUS_SCHEDULED):

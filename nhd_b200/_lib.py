@@ -15,7 +15,7 @@ EXPORTS = ('nhd_default_params', 'nhd_nccl_unique_id', 'nhd_shard_min_pairs', 'n
            'nhd_fetch_bindings', 'nhd_sync', 'nhd_run_filter_only', 'nhd_last_timing', 'nhd_read_filter',
            'nhd_debug_counters', 'nhd_alloc_pinned', 'nhd_free_pinned',
            'nhd_ingest_create', 'nhd_ingest_destroy', 'nhd_ingest_node', 'nhd_ingest_group_mask',
-           'nhd_ingest_speed_table', 'nhd_node_stats_from_records')
+           'nhd_ingest_speed_table', 'nhd_node_stats_from_records', 'nhd_explain')
 
 
 class Params(ctypes.Structure):
@@ -79,6 +79,7 @@ def load():
         'nhd_ingest_group_mask': (i32, [vp, ctypes.c_char_p, i32, ctypes.POINTER(ctypes.c_uint64)]),
         'nhd_ingest_speed_table': (i32, [vp, vp, ctypes.POINTER(i32)]),
         'nhd_node_stats_from_records': (i32, [i32, vp, vp]),
+        'nhd_explain': (i32, [vp, i32, vp, vp, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

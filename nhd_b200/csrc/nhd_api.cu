@@ -117,6 +117,12 @@ struct nhd_handle {
     uint64_t* d_pod_groups = nullptr; size_t pod_groups_cap = 0;
     std::vector<int32_t> pod_type_host;
 
+    /* nhd_explain's own buffers: the call leaves everything above as it was */
+    PodType* d_x_types = nullptr;   size_t x_types_cap = 0;
+    double* d_x_now = nullptr;      size_t x_now_cap = 0;
+    int32_t* d_x_out = nullptr;     size_t x_out_cap = 0;       /* counts [T][NHD_WHY_COUNT] | first [T][2] */
+    uint8_t* d_x_reasons = nullptr; size_t x_reasons_cap = 0;   /* [T][n_nodes] */
+
     nhd_timing timing;
     std::string err;
 };
@@ -300,6 +306,7 @@ extern "C" int32_t nhd_destroy(nhd_handle* h)
     cudaFree(h->d_prof);
 #endif
     cudaFree(h->d_pend); cudaFree(h->d_vresult); cudaFree(h->d_pod_groups);
+    cudaFree(h->d_x_types); cudaFree(h->d_x_now); cudaFree(h->d_x_out); cudaFree(h->d_x_reasons);
     if (h->h_stage) cudaFreeHost(h->h_stage);
     if (h->h_batch) cudaFreeHost(h->h_batch);
     if (h->h_out) cudaFreeHost(h->h_out);
@@ -577,10 +584,39 @@ static nhd_pod canonical_pod(const nhd_pod& in)
     return p;
 }
 
-extern "C" int32_t nhd_stage_batch(nhd_handle* h, int32_t n_pods, const nhd_pod* pods, const double* now)
+/* The checks every call that takes a batch of pods runs (nhd_stage_batch, nhd_explain): the arguments and the call
+ * order first, then each pod in order — its descriptor, its clock, the tuple limits of the loaded cluster. */
+static int32_t check_batch_args(nhd_handle* h, int32_t n_pods, const nhd_pod* pods, const double* now, const char* fn)
 {
     if (!h || n_pods < 0 || (n_pods > 0 && (!pods || !now))) return NHD_ERR_INVALID;
-    if (!h->loaded) return fail(h, NHD_ERR_STATE, "nhd_stage_batch before nhd_load_nodes");
+    if (!h->loaded) return fail(h, NHD_ERR_STATE, "%s before nhd_load_nodes", fn);
+    return NHD_OK;
+}
+
+static int32_t check_pod_clock(nhd_handle* h, int i, double now)
+{
+    if (!std::isfinite(now)) return fail(h, NHD_ERR_INVALID, "pod %d: non-finite clock", i);
+    return NHD_OK;
+}
+
+static int32_t check_pod(nhd_handle* h, int i, const nhd_pod& pod, double now)
+{
+    int32_t v = nhd_validate_pod(&pod);
+    if (v != NHD_OK) return fail(h, v, "pod %d: descriptor rejected by nhd_validate_pod", i);
+    v = check_pod_clock(h, i, now);
+    if (v != NHD_OK) return v;
+    if (!tuple_limits_ok(h->max_numa, pod.n_groups))
+        return fail(h, NHD_ERR_UNSUPPORTED, "pod %d: %d groups on %d-NUMA nodes exceeds the tuple limits", i,
+                    (int)pod.n_groups, h->max_numa);
+    return NHD_OK;
+}
+
+extern "C" int32_t nhd_stage_batch(nhd_handle* h, int32_t n_pods, const nhd_pod* pods, const double* now)
+{
+    {
+        const int32_t v = check_batch_args(h, n_pods, pods, now, "nhd_stage_batch");
+        if (v != NHD_OK) return v;
+    }
     CK(cudaSetDevice(h->params.device));
     h->staged = h->solved = false;
 
@@ -616,16 +652,13 @@ extern "C" int32_t nhd_stage_batch(nhd_handle* h, int32_t n_pods, const nhd_pod*
         }
         RawSlot& rs = raw_cache[rh & 255];
         if (rs.type >= 0 && rs.hash == rh && memcmp(&rs.raw, &pods[i], sizeof(nhd_pod)) == 0) {
-            if (!std::isfinite(now[i])) return fail(h, NHD_ERR_INVALID, "pod %d: non-finite clock", i);
+            const int32_t v = check_pod_clock(h, i, now[i]);
+            if (v != NHD_OK) return v;
             h->pod_type_host[i] = rs.type;
             continue;
         }
-        int32_t v = nhd_validate_pod(&pods[i]);
-        if (v != NHD_OK) return fail(h, v, "pod %d: descriptor rejected by nhd_validate_pod", i);
-        if (!std::isfinite(now[i])) return fail(h, NHD_ERR_INVALID, "pod %d: non-finite clock", i);
-        if (!tuple_limits_ok(h->max_numa, pods[i].n_groups))
-            return fail(h, NHD_ERR_UNSUPPORTED, "pod %d: %d groups on %d-NUMA nodes exceeds the tuple limits", i,
-                        (int)pods[i].n_groups, h->max_numa);
+        const int32_t v = check_pod(h, i, pods[i], now[i]);
+        if (v != NHD_OK) return v;
         PodKey k{canonical_pod(pods[i])};
         if (multi_group) k.p.group_mask = ~0ULL;
         auto it = index.find(k);
@@ -884,6 +917,107 @@ extern "C" int32_t nhd_read_filter(nhd_handle* h, int32_t* n_types, int32_t* wor
     if (pod_type) {
         if (n_pods < h->n_pods) return NHD_ERR_INVALID;
         memcpy(pod_type, h->pod_type_host.data(), (size_t)h->n_pods * 4);
+    }
+    return NHD_OK;
+}
+
+/* ------------------------------------------------------------------ explanation */
+
+/* Explain types: pods with the same canonical descriptor, group mask and clock get the same answer.  Unlike a batch
+ * with several group lists, the group gate is always part of the type (it is the first reason a node can have). */
+struct ExplainKey {
+    nhd_pod p;
+    double now;
+    bool operator==(const ExplainKey& o) const { return memcmp(this, &o, sizeof(ExplainKey)) == 0; }
+};
+struct ExplainKeyHash {
+    size_t operator()(const ExplainKey& k) const
+    {
+        uint64_t x;
+        memcpy(&x, &k.now, 8);
+        return PodKeyHash()(PodKey{k.p}) ^ (x * 0x9E3779B97F4A7C15ULL);
+    }
+};
+
+extern "C" int32_t nhd_explain(nhd_handle* h, int32_t n_pods, const nhd_pod* pods, const double* now,
+                               int32_t* counts, int32_t* first_fit, uint8_t* reasons)
+{
+    {
+        const int32_t v = check_batch_args(h, n_pods, pods, now, "nhd_explain");
+        if (v != NHD_OK) return v;
+    }
+    if (n_pods > 0 && !counts) return NHD_ERR_INVALID;
+    CK(cudaSetDevice(h->params.device));
+    std::unordered_map<ExplainKey, int32_t, ExplainKeyHash> index;
+    std::vector<PodType> types;
+    std::vector<double> tnow;
+    std::vector<int32_t> pod_type((size_t)n_pods);
+    for (int i = 0; i < n_pods; i++) {
+        const int32_t v = check_pod(h, i, pods[i], now[i]);
+        if (v != NHD_OK) return v;
+        ExplainKey k;
+        memset(&k, 0, sizeof(k));
+        k.p = canonical_pod(pods[i]);
+        k.now = now[i] + 0.0;                                    /* -0.0 -> +0.0 */
+        auto it = index.find(k);
+        if (it == index.end()) {
+            PodType t;
+            memset(&t, 0, sizeof(t));
+            make_pod_type(k.p, t);
+            it = index.emplace(k, (int32_t)types.size()).first;
+            types.push_back(t);
+            tnow.push_back(k.now);
+        }
+        pod_type[i] = it->second;
+    }
+    const int T = (int)types.size(), N = h->n_nodes;
+    if (T == 0) return NHD_OK;
+    std::vector<int32_t> out((size_t)T * (NHD_WHY_COUNT + 2));
+    std::vector<uint8_t> why;
+    if (N > 0) {
+        const size_t out_bytes = out.size() * 4;
+        CK(grow_dev(h->d_x_types, h->x_types_cap, (size_t)T * sizeof(PodType)));
+        CK(grow_dev(h->d_x_now, h->x_now_cap, (size_t)T * 8));
+        CK(grow_dev(h->d_x_out, h->x_out_cap, out_bytes));
+        if (reasons) CK(grow_dev(h->d_x_reasons, h->x_reasons_cap, (size_t)T * N));
+        int32_t* d_counts = h->d_x_out;
+        int32_t* d_first = h->d_x_out + (size_t)T * NHD_WHY_COUNT;
+        CK(cudaMemcpyAsync(h->d_x_types, types.data(), (size_t)T * sizeof(PodType), cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(h->d_x_now, tnow.data(), (size_t)T * 8, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemsetAsync(d_counts, 0, (size_t)T * NHD_WHY_COUNT * 4, h->stream));
+        CK(cudaMemsetAsync(d_first, 0x7F, (size_t)T * 2 * 4, h->stream));     /* 0x7F7F7F7F > any node: none yet */
+        ExplainArgs xa;
+        xa.nodes = h->d_nodes; xa.types = h->d_x_types; xa.now = h->d_x_now;
+        xa.n_types = T; xa.n_nodes = N;
+        xa.counts = d_counts; xa.first = d_first;
+        xa.reasons = reasons ? h->d_x_reasons : nullptr;
+        xa.min_busy = h->params.min_busy_secs;
+        memcpy(xa.cap, h->cap, sizeof(xa.cap));
+        for (int t0 = 0; t0 < T; t0 += 65535) {                  /* gridDim.y limit */
+            ExplainArgs xc = xa;
+            xc.types += t0; xc.now += t0; xc.counts += (size_t)t0 * NHD_WHY_COUNT; xc.first += (size_t)t0 * 2;
+            if (xc.reasons) xc.reasons += (size_t)t0 * N;
+            xc.n_types = std::min(T - t0, 65535);
+            explain_kernel<<<dim3((N + EXPLAIN_THREADS - 1) / EXPLAIN_THREADS, xc.n_types), EXPLAIN_THREADS, 0, h->stream>>>(xc);
+            CK(cudaGetLastError());
+        }
+        CK(cudaMemcpyAsync(out.data(), h->d_x_out, out_bytes, cudaMemcpyDeviceToHost, h->stream));
+        if (reasons) {
+            why.resize((size_t)T * N);
+            CK(cudaMemcpyAsync(why.data(), h->d_x_reasons, why.size(), cudaMemcpyDeviceToHost, h->stream));
+        }
+    }
+    CK(cudaStreamSynchronize(h->stream));
+    for (int i = 0; i < n_pods; i++) {
+        const int t = pod_type[i];
+        memcpy(counts + (size_t)i * NHD_WHY_COUNT, &out[(size_t)t * NHD_WHY_COUNT], NHD_WHY_COUNT * 4);
+        if (first_fit) {
+            /* Matcher.SelectNode (Matcher.py:412-420): a pod without GPUs prefers the first node without GPUs */
+            const int32_t any = out[(size_t)T * NHD_WHY_COUNT + 2 * t], nogpu = out[(size_t)T * NHD_WHY_COUNT + 2 * t + 1];
+            const int32_t pick = (!types[t].needs_gpu && nogpu < N) ? nogpu : any;
+            first_fit[i] = (N > 0 && pick < N) ? pick : -1;
+        }
+        if (reasons && N > 0) memcpy(reasons + (size_t)i * N, &why[(size_t)t * N], (size_t)N);
     }
     return NHD_OK;
 }

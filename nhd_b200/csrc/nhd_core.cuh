@@ -423,6 +423,57 @@ NHD_HD bool node_feasible(const nhd_node_rec& r, const PodType& t, const double*
 }
 
 /*
+ * Why FindNode drops node r for pod type t at clock now: the FIRST stage of the reference path that removes it
+ * (NHD_WHY_*, include/nhd_b200.h), NHD_WHY_FEASIBLE if none does.  The group test comes before the active test
+ * here, as in InitialNodeFilter (NHDScheduler.py:241-245), unlike node_gates.  The stages are the predicates
+ * node_feasible is built from: the GPU stage is non-empty iff some G-tuple passes gpu_ok, the CPU stage iff some
+ * (G+1)-tuple passes cpu_ok (Matcher.py:203-216: every tuple, not only those of the GPU stage), the NIC stage iff
+ * some G-tuple has a surviving entry without the PCIe pruning, the intersection (Matcher.py:349) iff one tuple
+ * passes all three, and the PCI-mode node survives iff that still holds with the pruning (:295-335).
+ */
+NHD_HD int node_reason(const nhd_node_rec& r, const PodType& t, const double* cap, double now, double min_busy)
+{
+    if ((r.group_mask & t.pod.group_mask) == 0) return NHD_WHY_NOT_IN_GROUP;
+    if (!(r.flags & NHD_NODE_ACTIVE)) return NHD_WHY_INACTIVE;
+    if (r.flags & NHD_NODE_MAINTENANCE) return NHD_WHY_MAINTENANCE;
+    if (t.pod.hugepages_gb > r.free_hugepages_gb) return NHD_WHY_HUGEPAGES;
+    if (!t.valid_map) return NHD_WHY_MAP_TYPE;
+    if (t.needs_gpu && node_busy(r, now, min_busy)) return NHD_WHY_BUSY;
+    const int K = r.n_numa, G = t.G;
+    int fg[NHD_MAX_NUMA], fc[NHD_MAX_NUMA];
+    free_gpus(r, fg);
+    free_cores(r, fc);
+    const bool smt = rec_smt(r);
+    /* 15 free GPUs on every switch: more than the <= NHD_MAX_GROUPS groups that can share one, so the PCI test of
+     * nic_first_fit always passes — the NIC stage as Matcher.FilterNumaTopology leaves it */
+    const uint64_t no_pruning = ~0ULL;
+    const uint64_t gsw = t.pci ? free_gpus_per_switch(r) : no_pruning;
+    bool any_gpu = false, any_cpu = false, any_nic = false, isect = false, isect_pruned = false;
+    const int np = ipow(K, G);
+    uint8_t p[NHD_MAX_GROUPS], idx[NHD_MAX_GROUPS], li[NHD_MAX_GROUPS];
+    for (int pi = 0; pi < np && !isect_pruned; pi++) {
+        tuple_digits(pi, K, G, p);
+        const bool g = gpu_ok(t, p, K, fg);
+        bool c = false;
+        for (int m = 0; m < K && !c; m++) c = cpu_ok(t, p, m, K, fc, smt);
+        any_gpu |= g;
+        any_cpu |= c;
+        if (any_nic && !(g && c)) continue;           /* nothing left to learn from this tuple's NICs */
+        const bool n = nic_first_fit(r, t, p, K, cap, no_pruning, idx, li);
+        any_nic |= n;
+        if (!(g && c && n)) continue;
+        isect = true;
+        isect_pruned = !t.pci || nic_first_fit(r, t, p, K, cap, gsw, idx, li);
+    }
+    if (!any_gpu) return NHD_WHY_GPU;
+    if (!any_cpu) return NHD_WHY_CPU;
+    if (!any_nic) return NHD_WHY_NIC;
+    if (!isect) return NHD_WHY_NUMA;
+    if (!isect_pruned) return NHD_WHY_PCIE;
+    return NHD_WHY_FEASIBLE;
+}
+
+/*
  * The same predicate for the common shape — a 2-NUMA node and a pod of one or two groups — written so that
  * nothing is indexed dynamically: the record, the per-NUMA counts and the search state all stay in registers
  * (node_feasible keeps its tuples, demand sums and NIC search stack in arrays, which the GPU puts in local

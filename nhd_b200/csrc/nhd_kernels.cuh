@@ -2470,4 +2470,55 @@ __global__ void commit_kernel(const FinishArgs a)
     *reinterpret_cast<double*>(a.nodes + chunk_off(node, 3)) = d.busy_time;
 }
 
+/* ------------------------------------------------------------------ explanation (nhd_explain) */
+
+constexpr int EXPLAIN_THREADS = 256;
+constexpr int EXPLAIN_NONE = 0x7FFFFFFF;          /* first-fit slot before any feasible node is seen */
+
+struct ExplainArgs {
+    const uint8_t* nodes;        /* tiled node array (read only) */
+    const PodType* types;        /* [n_types] explain types: descriptor with the pod's own group mask */
+    const double* now;           /* [n_types] clock of each explain type */
+    int n_types;
+    int n_nodes;
+    int32_t* counts;             /* [n_types][NHD_WHY_COUNT], zeroed by the caller */
+    int32_t* first;              /* [n_types][2]: first feasible node, first feasible node without GPUs (EXPLAIN_NONE) */
+    uint8_t* reasons;            /* [n_types][n_nodes] or null */
+    double min_busy;
+    double cap[NHD_MAX_SPEED_CLASSES];
+};
+
+/* One thread per (node, explain type): blockIdx.y = type, 32 consecutive nodes per warp, so each 16-byte chunk of
+ * the tiled records is one 512-byte coalesced read per warp.  Counts are summed per warp (one ballot per reason,
+ * one atomicAdd per warp and non-zero reason); first fit takes the lowest lane of a ballot, one atomicMin per warp.
+ * The node records are only read, and no buffer of the solve is touched. */
+__global__ void __launch_bounds__(EXPLAIN_THREADS)
+explain_kernel(const ExplainArgs a)
+{
+    const int t = blockIdx.y;
+    const int node = blockIdx.x * EXPLAIN_THREADS + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    const bool valid = node < a.n_nodes;
+    int why = -1;
+    bool nogpu = false;
+    if (valid) {
+        RecU u;
+        load_rec(a.nodes, node, u);
+        why = node_reason(u.r, a.types[t], a.cap, a.now[t], a.min_busy);
+        nogpu = u.r.n_gpus == 0;
+        if (a.reasons) a.reasons[(size_t)t * a.n_nodes + node] = (uint8_t)why;
+    }
+    const int base = node - lane;
+#pragma unroll
+    for (int w = 0; w < NHD_WHY_COUNT; w++) {
+        const uint32_t bal = __ballot_sync(0xFFFFFFFFu, why == w);
+        if (lane == 0 && bal) atomicAdd(&a.counts[t * NHD_WHY_COUNT + w], popc32(bal));
+        if (w == NHD_WHY_FEASIBLE) {
+            const uint32_t ng = __ballot_sync(0xFFFFFFFFu, why == w && nogpu);
+            if (lane == 0 && bal) atomicMin(&a.first[t * 2 + 0], base + ctz32(bal));
+            if (lane == 0 && ng) atomicMin(&a.first[t * 2 + 1], base + ctz32(ng));
+        }
+    }
+}
+
 } // namespace nhd

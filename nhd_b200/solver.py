@@ -167,6 +167,19 @@ class Solver:
         self._ck(self._L.nhd_debug_counters(self._h, out.ctypes.data))
         return out
 
+    def explain(self, pods, now, detail=False):
+        """Why each node is dropped for each pod, on the current records (``nhd_explain``; changes nothing).
+        Returns (counts[pod, WHY_COUNT] nodes per ``wire.WHY_*`` reason, first_fit[pod] the node FindNode would
+        pick now or -1, reasons[pod, node] uint8 codes when ``detail`` else None)."""
+        pods = np.ascontiguousarray(pods, dtype=wire.POD_DTYPE)
+        now = np.ascontiguousarray(np.broadcast_to(np.asarray(now, dtype='<f8'), (len(pods),)))
+        counts = np.zeros((len(pods), wire.WHY_COUNT), dtype='<i4')
+        first = np.zeros(len(pods), dtype='<i4')
+        reasons = np.zeros((len(pods), self.n_nodes), dtype=np.uint8) if detail else None
+        self._ck(self._L.nhd_explain(self._h, len(pods), pods.ctypes.data, now.ctypes.data, counts.ctypes.data,
+                                     first.ctypes.data, reasons.ctypes.data if detail else None))
+        return counts, first, reasons
+
     def filter_bitmaps(self):
         """Runs only the snapshot predicate kernel on the staged batch; returns
         (feas[type, node] bool, nogpu[node], busy[node], pod_type[pod])."""

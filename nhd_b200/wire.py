@@ -22,6 +22,18 @@ PLACED, NO_CANDIDATE, ASSIGN_FAILED, REF_WOULD_CRASH, BAD_MAP_TYPE = 0, 1, 2, 3,
 STATUS_NAMES = {PLACED: 'placed', NO_CANDIDATE: 'none', ASSIGN_FAILED: 'assign_failed',
                 REF_WOULD_CRASH: 'ref_would_crash', BAD_MAP_TYPE: 'bad_map_type'}
 
+# nhd_explain reason codes (NHD_WHY_*): the first stage of the reference path that drops a node for a pod
+(WHY_FEASIBLE, WHY_NOT_IN_GROUP, WHY_INACTIVE, WHY_MAINTENANCE, WHY_HUGEPAGES, WHY_MAP_TYPE, WHY_BUSY, WHY_GPU, WHY_CPU,
+ WHY_NIC, WHY_PCIE, WHY_NUMA) = range(12)
+WHY_COUNT = 12
+WHY_NAMES = ('FEASIBLE', 'NOT_IN_GROUP', 'INACTIVE', 'MAINTENANCE', 'HUGEPAGES', 'MAP_TYPE', 'BUSY', 'GPU', 'CPU',
+             'NIC', 'PCIE', 'NUMA')
+# short text per code, in the style of kube-scheduler's "0/N nodes are available: 3 <text>, ..."
+WHY_TEXT = ('feasible', "not in the pod's node groups", 'inactive', 'in maintenance', 'too few free hugepages',
+            'unsupported topology map type', 'busy after a recent GPU deployment', 'too few free GPUs per NUMA node',
+            'too few free CPU cores', 'too little free NIC bandwidth', 'no NIC on a PCIe switch with a free GPU',
+            'GPUs, CPU cores and NICs on different NUMA nodes')
+
 MAP_INVALID, MAP_NUMA, MAP_PCI, MAP_NONE = 0, 1, 2, 3
 NODE_SMT, NODE_ACTIVE, NODE_MAINTENANCE = 1, 2, 4
 GRP_PROC_SMT, GRP_HELPER_SMT, GRP_HAS_NIC_CORES = 1, 2, 4
